@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 3                      # this repo's CUDA path
     torchrun --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 3 --warmup 1               # the reference's CPU path on the host cores
+    python bench.py --steps 20 --warmup 3 --dump-outputs DIR            # + the last timed generation's outputs as DIR/*.npy
 
 A "step" is one generation over synthetic input: draw K noise indices -> theta +- sigma*eps ->
 open-loop MLP rollouts (T steps) -> fitness -> [allgather] -> centered rank -> sum_k w_k eps_k ->
@@ -70,7 +71,15 @@ def parse(argv=None):
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-also', action='store_true', help='headline only (skip modes / parity / strong-scaling side measurements)')
-    return ap.parse_args(argv)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the headline generation computed in its last timed step as DIR/<name>.npy (float32 / '
+                         'float64, at most 64 MB): the same arguments give the same inputs, so two builds compare array by array')
+    args = ap.parse_args(argv)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
+    return args
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -315,6 +324,39 @@ def float64_truth_report(gen, modes, torch):
     return out
 
 
+DUMP_BYTES = 60_000_000                 # under 64 MB with the .npy headers
+DUMP_SAMPLE = 1 << 18
+
+
+def generation_outputs(gen) -> dict:
+    """What one ``DeviceGeneration.run`` hands its caller, as host arrays: the updated parameters, both fitness signs and
+    the noise indices of all K pairs (rank-major), this process's rank weights and the generation's obs statistics."""
+    import numpy as np
+    multi = gen.comm.size > 1
+    dev = dict(theta=gen.theta, fitness_pos=gen.fpos_all if multi else gen.fit_local[0],
+               fitness_neg=gen.fneg_all if multi else gen.fit_local[1], noise_idx=gen.idx_all if multi else gen.idx,
+               rank_weights=gen.weights, obs_sum=gen.gen_sum, obs_sumsq=gen.gen_sumsq, obs_count=gen.gen_count)
+    out = {}
+    for name, t in dev.items():
+        a = t.detach().cpu().numpy()
+        out[name] = a.astype(np.float64 if a.dtype in (np.float64, np.int64) else np.float32)   # indices < 2^53: exact
+    return out
+
+
+def dump_outputs(arrays: dict, folder: str):
+    """np.save every array; when together they exceed DUMP_BYTES, arrays longer than DUMP_SAMPLE elements are replaced by a
+    fixed seeded sample of their flattened elements and the sampled positions are written as <name>_sample_index.npy."""
+    import numpy as np
+    os.makedirs(folder, exist_ok=True)
+    sample = sum(a.nbytes for a in arrays.values()) > DUMP_BYTES
+    for name, a in arrays.items():
+        if sample and a.size > DUMP_SAMPLE:
+            pick = np.sort(np.random.RandomState(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            np.save(os.path.join(folder, f'{name}_sample_index.npy'), pick.astype(np.float64))
+            a = a.reshape(-1)[pick]
+        np.save(os.path.join(folder, f'{name}.npy'), a)
+
+
 def run_ours(args, wl, n_gpus):
     import numpy as np
     import torch
@@ -368,9 +410,9 @@ def run_ours(args, wl, n_gpus):
                                 save_obs_chance=0.01, rollout_mode=MODE_ID[mode_name], comm=comm, engine=eng,
                                 archive=None if archive is None else eng.to_device(archive, torch.float64), nov_k=10, moo_w=0.5, **kw)
 
-    def measure(gen, pairs_local, steps, warmup, sampler=None):
+    def measure(gen, pairs_local, steps, warmup, sampler=None, outputs=None):
         """K-generation timing of ``gen`` at ``pairs_local`` pairs per GPU: max-over-ranks ms per step + per-kernel event
-        means of the timed steps + launches."""
+        means of the timed steps + launches.  ``outputs`` (a dict) receives generation_outputs(gen) of the last timed step."""
         nps = pairs_local // gen.n_streams
         state = {}
 
@@ -383,6 +425,8 @@ def run_ours(args, wl, n_gpus):
         def on_end():
             state['launches'] = eng.launches - state['l0']
             state['timers'], gen.timers = gen.timers, None          # no event pairs for the untimed continuation
+            if outputs is not None:
+                outputs.update(generation_outputs(gen))
 
         max_s, extra = timed_region(lambda: gen.run(nps), steps, warmup, comm, torch.cuda.synchronize, _EventTimer(torch),
                                     allreduce_max, min_load_s=0.6 if sampler is not None else 0.0,
@@ -393,7 +437,8 @@ def run_ours(args, wl, n_gpus):
     # ---------------- device-resident generation: `value` (headline config, headline mode) ----------------
     gen = make_gen(head_mode, bool(wl.get('nsra')))
     sampler = ClockSampler(local)
-    head = measure(gen, k_local, args.steps, args.warmup, sampler)
+    head_outputs = {} if (args.dump_outputs and rank == 0) else None
+    head = measure(gen, k_local, args.steps, args.warmup, sampler, head_outputs)
     clocks = sampler.stop() if rank == 0 else None
     if clocks is not None:
         clocks['window'] = f'timed region ({args.steps} steps) + {head["extra"]} untimed identical generations'
@@ -531,6 +576,8 @@ def run_ours(args, wl, n_gpus):
 
     if rank != 0:
         return
+    if head_outputs is not None:
+        dump_outputs(head_outputs, args.dump_outputs)
     peaks = {}
     try:
         with open(os.path.join(ROOT, 'MEASURED_PEAKS.json')) as f:

@@ -5,8 +5,8 @@ GPU, and under torchrun on two -- with the settings the shipped configs use (ac_
 generation is replayed by the CPU oracle: indices and the ranks' RandomState streams bit-exact, fitness to float32
 tolerance, theta within 1e-5 after three generations of Adam.
 
-(The reference's own scripts cannot be executed where a GPU is: /root/reference exists only in the build container, which
-has no GPU; tests/test_host_logic.py checks there that they import against the same shims.)"""
+(The reference's own scripts are not part of this repository; tests/test_host_logic.py checks that their import statements,
+recorded in tests/golden/ref_script_surface.json, resolve against the same shims.)"""
 import json
 import os
 import socket

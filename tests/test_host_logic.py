@@ -2,6 +2,7 @@
 host-side mirror keeps the reference's API surface, the shims let the reference scripts import,
 and the multi-process plumbing (gloo, world_size 2) keeps the reference's result layout."""
 import importlib.util
+import json
 import os
 import re
 import subprocess
@@ -140,25 +141,34 @@ def test_policy_flat_layout_and_pickle(tmp_path):
     assert np.array_equal(pol2.flat_params, pol.flat_params) and pol2.optim.t == 0 and pol2.std == 0.02
 
 
-def test_reference_scripts_import_against_the_shims():
-    """simple_example.py / obj.py / nsra.py / multi_agent.py resolve every import against es_pytorch_b200/compat
-    (only where the reference checkout is mounted: the build container)."""
-    if not os.path.isdir('/root/reference'):
-        pytest.skip('reference checkout not present on this box')
+def test_reference_scripts_import_against_the_shims(tmp_path):
+    """Every import statement of simple_example.py / obj.py / nsra.py / multi_agent.py (their module-level code is imports
+    and function definitions) resolves against es_pytorch_b200/compat, and the shims' load_config reads
+    configs/simple_conf.json; both recorded from the reference by tests/golden/make_ref_cases.py."""
+    with open(os.path.join(ROOT, 'tests', 'golden', 'ref_script_surface.json')) as f:
+        surface = json.load(f)
+    assert sorted(surface['imports']) == ['multi_agent', 'nsra', 'obj', 'simple_example']
+    conf = tmp_path / 'simple_conf.json'
+    conf.write_text(json.dumps(surface['simple_conf']))
     code = textwrap.dedent('''
-        import importlib.util, sys
-        for s in ('simple_example', 'obj', 'nsra', 'multi_agent'):
-            spec = importlib.util.spec_from_file_location('ref_' + s, '/root/reference/%s.py' % s)
-            m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
+        import json, sys
+        surface = json.load(open(sys.argv[1]))
+        for script, rows in surface['imports'].items():
+            for row in rows:
+                if 'names' in row:
+                    exec('from %s import %s' % (row['module'], ', '.join(row['names'])), {})
+                else:
+                    exec('import ' + row['module'], {})
         import src.core.es, es_pytorch_b200.core.es
         assert src.core.es is es_pytorch_b200.core.es
         from src.utils import utils
-        cfg = utils.load_config('/root/reference/configs/simple_conf.json')
+        cfg = utils.load_config(sys.argv[2])
         assert cfg.general.policies_per_gen == 4800 and cfg.noise.std == 0.02
         print('OK')
     ''')
     env = dict(os.environ, PYTHONPATH=ROOT + os.pathsep + COMPAT)
-    out = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, env=env)
+    out = subprocess.run([sys.executable, '-c', code, os.path.join(ROOT, 'tests', 'golden', 'ref_script_surface.json'), str(conf)],
+                         capture_output=True, text=True, env=env)
     assert out.returncode == 0 and 'OK' in out.stdout, out.stderr[-2000:]
 
 

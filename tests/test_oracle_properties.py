@@ -1,18 +1,14 @@
 """CPU property tests (hypothesis): the oracle's restatements against live third-party / reference behaviour on random inputs,
 beyond the fixed golden vectors.
   * the MT19937 + masked-rejection restatement against numpy's legacy RandomState (the pinned RNG of the reference);
-  * the rank shapings against the REAL reference module when /root/reference is present (the build container; skipped on
-    the GPU box, where only the committed golden vectors travel)."""
+  * the rank shapings and EliteRanker against outputs of the REAL reference module on 120 seeded random cases
+    (tests/golden/ref_ranker_cases.npz, written by tests/golden/make_ref_cases.py)."""
 import os
-import sys
 
 import numpy as np
-import pytest
 from hypothesis import given, settings, strategies as st
 
 from oracle import es_oracle as orc
-
-REF = '/root/reference'
 
 
 @settings(max_examples=25, deadline=None)
@@ -37,46 +33,33 @@ def test_mt_draw_restatement_matches_numpy_legacy_randomstate(seed, burn, n, ub,
     assert [int(cont.randint(0, 1 << 30)) for _ in range(5)] == [int(rs.randint(0, 1 << 30)) for _ in range(5)]
 
 
-def _ref_rankers():
-    if not os.path.isdir(os.path.join(REF, 'src', 'utils')):
-        pytest.skip('reference checkout not present (GPU box): the committed golden vectors cover this')
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    from src.utils import rankers as R
-    return R
+def _ranker_cases():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'ref_ranker_cases.npz'))
 
 
-finite = st.floats(min_value=-1e6, max_value=1e6, allow_nan=False, allow_infinity=False, width=64)
+def test_shapings_match_the_real_reference_rankers():
+    v = _ranker_cases()
+    off = v['shape_off']
+    for i, code in enumerate(v['shape_name']):
+        name = str(v['shapings'][code])
+        x = v['shape_x'][off[i]:off[i + 1]].reshape(-1, 1)
+        k = len(x) // 2
+        want = v['shape_w'][off[i] // 2:off[i + 1] // 2].astype(v['shape_w_dtype'][i]).reshape((k,) if v['shape_w_ndim'][i] == 1 else (k, 1))
+        got, n = orc.shaped_ranker(x[:k], x[k:], name)
+        assert n == 2 * k and got.dtype == want.dtype and got.shape == want.shape, (i, name)
+        assert np.array_equal(got, want, equal_nan=True), (i, name)
 
 
-@settings(max_examples=40, deadline=None)
-@given(data=st.data(), k=st.integers(1, 40), name=st.sampled_from(['centered', 'double_positive', 'semi_centered', 'max_normalized']))
-def test_shapings_match_the_real_reference_rankers(data, k, name):
-    R = _ref_rankers()
-    cls = {'centered': R.CenteredRanker, 'double_positive': R.DoublePositiveCenteredRanker,
-           'semi_centered': R.SemiCenteredRanker, 'max_normalized': R.MaxNormalizedRanker}[name]
-    vals = data.draw(st.lists(finite, min_size=2 * k, max_size=2 * k, unique=True))     # tie order is unpinned in the reference
-    x = np.array(vals, dtype=np.float64).reshape(2 * k, 1)
-    pos, neg = x[:k], x[k:]
-    if name == 'max_normalized' and (x.max() + (-x.min() if x.min() > 0 else x.min())) == 0:
-        return                                                                            # the reference divides by zero
-    want = cls().rank(pos.copy(), neg.copy(), np.arange(k))
-    got, n = orc.shaped_ranker(pos, neg, name)
-    assert n == 2 * k and got.dtype == want.dtype and got.shape == want.shape
-    assert np.array_equal(got, want, equal_nan=True)
-
-
-@settings(max_examples=40, deadline=None)
-@given(data=st.data(), k=st.integers(1, 40), pct=st.floats(0, 1), name=st.sampled_from(['centered', 'double_positive']))
-def test_elite_matches_the_real_reference_ranker(data, k, pct, name):
-    R = _ref_rankers()
-    cls = {'centered': R.CenteredRanker, 'double_positive': R.DoublePositiveCenteredRanker}[name]
-    vals = data.draw(st.lists(finite, min_size=2 * k, max_size=2 * k, unique=True))
-    x = np.array(vals, dtype=np.float64).reshape(2 * k, 1)
-    inds = np.arange(100, 100 + k).astype(np.float64)
-    e = R.EliteRanker(cls(), pct)
-    want = np.asarray(e.rank(x[:k].copy(), x[k:].copy(), inds.copy()))
-    vals_o, inds_o, _, n = orc.elite_ranker(x[:k], x[k:], inds, name, pct)
-    assert n == e.n_fits_ranked == len(want)
-    a, b = np.lexsort((e.noise_inds, want)), np.lexsort((inds_o, vals_o))            # argpartition's order is unspecified
-    assert np.array_equal(want[a], vals_o[b]) and np.array_equal(np.asarray(e.noise_inds)[a], inds_o[b])
+def test_elite_matches_the_real_reference_ranker():
+    v = _ranker_cases()
+    off, off_out = v['elite_off'], v['elite_off_out']
+    for i, code in enumerate(v['elite_name']):
+        name = str(v['shapings'][code])
+        x = v['elite_x'][off[i]:off[i + 1]].reshape(-1, 1)
+        k = len(x) // 2
+        want, want_inds = v['elite_vals'][off_out[i]:off_out[i + 1]], v['elite_inds'][off_out[i]:off_out[i + 1]]
+        inds = np.arange(100, 100 + k).astype(np.float64)
+        vals_o, inds_o, _, n = orc.elite_ranker(x[:k], x[k:], inds, name, float(v['elite_pct'][i]))
+        assert n == len(want), (i, name)
+        b = np.lexsort((inds_o, vals_o))                                                  # argpartition's order is unspecified
+        assert np.array_equal(want, vals_o[b]) and np.array_equal(want_inds, inds_o[b]), (i, name)
