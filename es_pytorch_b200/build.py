@@ -17,8 +17,8 @@ CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libes_b200.so')
 STAMP = os.path.join(HERE, '.libes_b200.stamp')
 
-SOURCES = ['api.cu', 'reconstruct.cu', 'rank.cu', 'elementwise.cu', 'mt_draw.cu', 'mt_gauss.cu', 'rollout_f32.cu', 'rollout_f32x.cu', 'rollout_tc2.cu', 'rollout_closed.cu']
-HEADERS = ['common.cuh', 'mt19937.cuh', 'mt_jump_polys.inc', os.path.join('..', '..', 'include', 'es_b200.h')]
+SOURCES = ['api.cu', 'reconstruct.cu', 'rank.cu', 'elementwise.cu', 'mt_draw.cu', 'mt_gauss.cu', 'rollout_f32.cu', 'rollout_f32x.cu', 'rollout_tc2.cu', 'rollout_tcw.cu', 'rollout_closed.cu']
+HEADERS = ['common.cuh', 'tc_ptx.cuh', 'mt19937.cuh', 'mt_jump_polys.inc', os.path.join('..', '..', 'include', 'es_b200.h')]
 
 NVCC_FLAGS = [
     '-gencode', 'arch=compute_100a,code=sm_100a',

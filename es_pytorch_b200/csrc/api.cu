@@ -230,10 +230,23 @@ int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len
         return es_impl_rollout_f32(ctx, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers, obsn,
                                    rew_vec, T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg,
                                    act_noise, (cudaStream_t)stream);
-    if (mode == ES_ROLLOUT_TC || mode == ES_ROLLOUT_TC3)
+    if (mode == ES_ROLLOUT_TC || mode == ES_ROLLOUT_TC3) {
+        // obs-64-64-act: rollout_tc2.cu (layer 1 shared by both signs through U +- sigma V); 2..4 hidden layers of 64..256
+        // (multiples of 64): rollout_tcw.cu (per-pair weight images streamed through shared memory)
+        const bool h64 = n_layers == 3 && layer_sizes[1] == 64 && layer_sizes[2] == 64;
+        if (!h64 && es_tcw_covers(layer_sizes, n_layers))
+            return es_impl_rollout_tcw(ctx, mode == ES_ROLLOUT_TC3, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes,
+                                       n_layers, obsn, rew_vec, T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg,
+                                       act_noise, (cudaStream_t)stream);
+        if (!h64) {
+            es_set_error("es_rollout_openloop(TC): the tensor-core path covers tanh MLPs obs(<=1023) -> 2..4 hidden layers "
+                         "(each a multiple of 64 in [64, 256]) -> act(<=32); use ES_ROLLOUT_F32 for other shapes");
+            return ES_ERR_UNSUPPORTED;
+        }
         return es_impl_rollout_tc2(ctx, mode == ES_ROLLOUT_TC3, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers,
                                    obsn, rew_vec, T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg,
                                    act_noise, (cudaStream_t)stream);
+    }
     es_set_error("es_rollout_openloop: unknown mode %d", mode);
     return ES_ERR_INVALID;
 }

@@ -93,6 +93,10 @@ int es_impl_rollout_tc2(es_ctx*, int split, const float*, int64_t, const int64_t
                         int, const float*, const float*, int, float, double*, double*, int, float*, float*, const float*,
                         cudaStream_t);
 void es_tc2_free_shadows(es_ctx* ctx);
+int es_impl_rollout_tcw(es_ctx*, int split, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*,
+                        int, const float*, const float*, int, float, double*, double*, int, float*, float*, const float*,
+                        cudaStream_t);
+int es_tcw_covers(const int* layer_sizes, int n_layers);      // shapes of rollout_tcw.cu
 int es_impl_rollout_closed(es_ctx*, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*, const double*,
                            const double*, double, const float*, const float*, int, const float*, const float*, int, float,
                            const uint32_t*, double, double*, double*, int, float*, float*, double*, double*, double*, cudaStream_t);

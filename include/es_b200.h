@@ -100,7 +100,10 @@ int es_normalise_obs(es_ctx* ctx, const float* obs, const double* mean, const do
  *                          population spread of the float32 result, see DESIGN.md)
  *         ES_ROLLOUT_TC3 = tcgen05 tensor-core path at float32-equivalent accuracy: every operand is split into
  *                          float16 hi + lo parts and every product is three MMAs (hi*hi + hi*lo + lo*hi), float32
- *                          accumulation in TMEM, accurate tanh, float64 fitness sums (see DESIGN.md)                */
+ *                          accumulation in TMEM, accurate tanh, float64 fitness sums (see DESIGN.md)
+ *         The tensor-core modes cover tanh MLPs with obs_dim <= 1023, act_dim <= 32 and either two hidden layers of 64
+ *         (rollout_tc2.cu) or 2 to 4 hidden layers, each a multiple of 64 in [64, 256] (rollout_tcw.cu: the networks of
+ *         the shipped configs); other shapes return ES_ERR_UNSUPPORTED.                                              */
 #define ES_ROLLOUT_F32 0
 #define ES_ROLLOUT_TC  1
 #define ES_ROLLOUT_TC3 2
