@@ -38,6 +38,8 @@ SIGNATURES = {
                                    _f32, _vp, _vp, _i32, _vp, _vp, _i32, _vp]),
     'es_rollout_openloop_noisy': (_i32, [_vp, _vp, _i64, _vp, _i32, _vp, _i32, _f32, C.POINTER(_i32), _i32, _vp, _vp, _i32,
                                          _f32, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _vp]),
+    'es_rollout_openloop_episodes': (_i32, [_vp, _vp, _i64, _vp, _i32, _vp, _i32, _f32, C.POINTER(_i32), _i32, _vp, _vp, _i32,
+                                            _f32, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _vp]),
     'es_rollout_closedloop': (_i32, [_vp, _vp, _i64, _vp, _i32, _vp, _i32, _f32, C.POINTER(_i32), _i32, _vp, _vp, _f64, _vp, _vp, _i32,
                                      _vp, _vp, _i32, _f32, _vp, _f64, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     'es_draw_noisy': (_i32, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _u64, _i32, _i32, _f64, _vp, _vp, _vp, _vp]),

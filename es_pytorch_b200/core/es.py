@@ -175,7 +175,8 @@ def _device_generation(fit_fn, policy: Policy, nt: NoiseTable, streams) -> Devic
     theta = policy.theta_dev(eng)
     if (gen is None or gen.theta is not theta or gen.n_streams != len(streams) or gen.table is not nt.device_table(eng)
             or gen.coins_per_eval != int(fit_fn.coins_per_eval) or gen.rollout_mode != fit_fn.rollout_mode
-            or (gen.archive is None) != (fit_fn.archive is None)):
+            or (gen.archive is None) != (fit_fn.archive is None)
+            or gen.eps_per_policy != getattr(fit_fn, 'eps_per_policy', 1)):
         env = fit_fn.env
         obs_dev, rew_dev = env.device_arrays(eng)
         T = fit_fn.max_steps
@@ -186,7 +187,8 @@ def _device_generation(fit_fn, policy: Policy, nt: NoiseTable, streams) -> Devic
                                coins_per_eval=fit_fn.coins_per_eval, save_obs_chance=fit_fn.save_obs_chance,
                                archive=archive, nov_k=fit_fn.nov_k, rollout_mode=fit_fn.rollout_mode, engine=eng,
                                ac_std=float(getattr(policy._module, '_action_std', 0.0) or 0.0),
-                               closed=env.device_closed(eng) if getattr(env, 'is_synthetic_closedloop', False) else None)
+                               closed=env.device_closed(eng) if getattr(env, 'is_synthetic_closedloop', False) else None,
+                               eps_per_policy=getattr(fit_fn, 'eps_per_policy', 1))
         fit_fn._gen = gen
     else:
         gen.load_states(streams)

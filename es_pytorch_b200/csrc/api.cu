@@ -207,11 +207,11 @@ int es_obstat_accumulate_coins(es_ctx* ctx, double* sum, double* sumsq, double* 
                                            n_coins, chance, (cudaStream_t)stream);
 }
 
-int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
-                              const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
-                              const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
-                              float* behv_pos, float* behv_neg, const float* act_noise, int mode, void* stream) {
-    ES_ENTER(ctx);
+// es_rollout_openloop_noisy (n_episodes = 1) and es_rollout_openloop_episodes: validation and dispatch
+static int rollout_openloop(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
+                            const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
+                            const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
+                            float* behv_pos, float* behv_neg, const float* act_noise, int n_eps, int mode, cudaStream_t stream) {
     ES_REQUIRE(table && idx && theta && layer_sizes && obsn && rew_vec && fit_pos && fit_neg,
                "es_rollout_openloop: NULL pointer");
     ES_REQUIRE(n_layers >= 1 && n_layers <= ES_MAX_LAYERS, "es_rollout_openloop: n_layers must be in [1,%d]",
@@ -225,11 +225,16 @@ int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len
     }
     ES_REQUIRE(count == P, "es_rollout_openloop: layer sizes give %lld params, P=%d", (long long)count, P);
     ES_REQUIRE(table_len > P, "es_rollout_openloop: table smaller than the network");
+    ES_REQUIRE(n_eps >= 1, "es_rollout_openloop_episodes: n_episodes must be >= 1, got %d", n_eps);
+    if (!act_noise) n_eps = 1;          // noise-free episodes are all the same episode: their average is its reward, exactly
+    ES_REQUIRE(n_eps == 1 || (int64_t)n_eps * T * layer_sizes[n_layers] <= 0x7FFFFFFF,
+               "es_rollout_openloop_episodes: n_episodes * T * act_dim = %lld exceeds INT_MAX (es_draw_noisy's normals_per_eval)",
+               (long long)n_eps * T * layer_sizes[n_layers]);
     if (n_pairs == 0) return ES_OK;
     if (mode == ES_ROLLOUT_F32)
         return es_impl_rollout_f32(ctx, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers, obsn,
                                    rew_vec, T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg,
-                                   act_noise, (cudaStream_t)stream);
+                                   act_noise, n_eps, stream);
     if (mode == ES_ROLLOUT_TC || mode == ES_ROLLOUT_TC3) {
         // obs-64-64-act: rollout_tc2.cu (layer 1 shared by both signs through U +- sigma V); 2..4 hidden layers of 64..256
         // (multiples of 64): rollout_tcw.cu (per-pair weight images streamed through shared memory)
@@ -237,7 +242,7 @@ int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len
         if (!h64 && es_tcw_covers(layer_sizes, n_layers))
             return es_impl_rollout_tcw(ctx, mode == ES_ROLLOUT_TC3, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes,
                                        n_layers, obsn, rew_vec, T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg,
-                                       act_noise, (cudaStream_t)stream);
+                                       act_noise, n_eps, stream);
         if (!h64) {
             es_set_error("es_rollout_openloop(TC): the tensor-core path covers tanh MLPs obs(<=1023) -> 2..4 hidden layers "
                          "(each a multiple of 64 in [64, 256]) -> act(<=32); use ES_ROLLOUT_F32 for other shapes");
@@ -245,10 +250,28 @@ int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len
         }
         return es_impl_rollout_tc2(ctx, mode == ES_ROLLOUT_TC3, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers,
                                    obsn, rew_vec, T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg,
-                                   act_noise, (cudaStream_t)stream);
+                                   act_noise, n_eps, stream);
     }
     es_set_error("es_rollout_openloop: unknown mode %d", mode);
     return ES_ERR_INVALID;
+}
+
+int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
+                              const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
+                              const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
+                              float* behv_pos, float* behv_neg, const float* act_noise, int mode, void* stream) {
+    ES_ENTER(ctx);
+    return rollout_openloop(ctx, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers, obsn, rew_vec, T, pos_scale,
+                            fit_pos, fit_neg, fit_stride, behv_pos, behv_neg, act_noise, 1, mode, (cudaStream_t)stream);
+}
+
+int es_rollout_openloop_episodes(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
+                                 const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
+                                 const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
+                                 float* behv_pos, float* behv_neg, const float* act_noise, int n_episodes, int mode, void* stream) {
+    ES_ENTER(ctx);
+    return rollout_openloop(ctx, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers, obsn, rew_vec, T, pos_scale,
+                            fit_pos, fit_neg, fit_stride, behv_pos, behv_neg, act_noise, n_episodes, mode, (cudaStream_t)stream);
 }
 
 int es_rollout_openloop(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,

@@ -84,17 +84,20 @@ int es_impl_obstat_accumulate_coins(es_ctx*, double*, double*, double*, const fl
                                     const uint32_t*, int, double, cudaStream_t);
 int es_impl_draw_noisy(es_ctx*, uint32_t*, int32_t*, int32_t*, double*, int, int, uint64_t, int, int, double, int64_t*, uint32_t*,
                        float*, cudaStream_t);
-// (the trailing const float* of the rollouts: scaled action noise [n_pairs][2][T][act], or NULL)
+// (the trailing const float*, int of the rollouts: scaled action noise [n_pairs][2][n_eps][T][act], or NULL, and the number
+// of episodes per evaluation n_eps; n_eps > 1 only with noise)
 int es_impl_rollout_f32(es_ctx*, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*, int,
-                        const float*, const float*, int, float, double*, double*, int, float*, float*, const float*, cudaStream_t);
+                        const float*, const float*, int, float, double*, double*, int, float*, float*, const float*, int,
+                        cudaStream_t);
 int es_impl_rollout_f32x(es_ctx*, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*, int,
-                         const float*, const float*, int, float, double*, double*, int, float*, float*, const float*, cudaStream_t);
+                         const float*, const float*, int, float, double*, double*, int, float*, float*, const float*, int,
+                         cudaStream_t);
 int es_impl_rollout_tc2(es_ctx*, int split, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*,
-                        int, const float*, const float*, int, float, double*, double*, int, float*, float*, const float*,
+                        int, const float*, const float*, int, float, double*, double*, int, float*, float*, const float*, int,
                         cudaStream_t);
 void es_tc2_free_shadows(es_ctx* ctx);
 int es_impl_rollout_tcw(es_ctx*, int split, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*,
-                        int, const float*, const float*, int, float, double*, double*, int, float*, float*, const float*,
+                        int, const float*, const float*, int, float, double*, double*, int, float*, float*, const float*, int,
                         cudaStream_t);
 int es_tcw_covers(const int* layer_sizes, int n_layers);      // shapes of rollout_tcw.cu
 int es_impl_rollout_closed(es_ctx*, const float*, int64_t, const int64_t*, int, const float*, int, float, const int*, const double*,

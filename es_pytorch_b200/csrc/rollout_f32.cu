@@ -102,15 +102,17 @@ rollout_f32_stage_kernel(const float* __restrict__ table, const int64_t* __restr
     rf_stage_weights(W, table + es_checked_slice(idx[blockIdx.x >> 1], d.P, d.table_len, d.err), theta, sigma, blockIdx.x & 1, d);
 }
 
-// GW: weights in the global scratch filled by rollout_f32_stage_kernel instead of shared memory
-template <bool GW>
+// GW: weights in the global scratch filled by rollout_f32_stage_kernel instead of shared memory.
+// EPIS: n_eps > 1 episodes per evaluation (act_noise [2*pair + sign][n_eps][T][act]); the forward pass is shared, every episode
+// adds its own noise row (the actions in xin stay noise-free) and the last episode drives the position integrator
+template <bool GW, bool EPIS>
 __global__ void __launch_bounds__(RF_THREADS, 1)
 rollout_f32_kernel(const float* __restrict__ table, const int64_t* __restrict__ idx, const float* __restrict__ theta,
                    float sigma, const __grid_constant__ RfDesc d, const float* __restrict__ obsn,
                    const float* __restrict__ rew_vec, int T, float pos_scale, double* __restrict__ fit_pos,
                    double* __restrict__ fit_neg, int fit_stride, float* __restrict__ behv_pos,
                    float* __restrict__ behv_neg, double* __restrict__ part, unsigned* __restrict__ tickets,
-                   const float* __restrict__ wglobal, const float* __restrict__ act_noise) {
+                   const float* __restrict__ wglobal, const float* __restrict__ act_noise, int n_eps) {
     extern __shared__ __align__(16) float smem[];
     float* Wsm = GW ? const_cast<float*>(wglobal) + (size_t)blockIdx.x * d.w_floats : smem;    // [w_floats]
     float* Xa = GW ? smem : smem + d.w_floats;          // [RF_TM][xpitch]
@@ -162,6 +164,41 @@ rollout_f32_kernel(const float* __restrict__ table, const int64_t* __restrict__ 
             float* tmp = xin; xin = xout; xout = tmp;
         }
         // xin now holds the actions [RF_TM][act_dim]
+        if (EPIS) {
+            // obj.py's episode loop: per step, the float32 reward of every episode's noisy action summed in float64 (the
+            // reference's rews[t] += r before the division by E, done once at the end)
+            __shared__ double s_rew_e[RF_TM];
+            __shared__ float s_last[RF_TM][3];              // the last episode's noisy action components 0, 1 % act, 2 % act
+            if (threadIdx.x < rows) {
+                const int r = threadIdx.x;
+                const float* a = xin + r * d.xpitch;
+                const float* c = rew_vec + (size_t)(t0 + r) * act_dim;
+                double racc = 0.0;
+                for (int e = 0; e < n_eps; ++e) {
+                    const float* __restrict__ nz = act_noise + (((size_t)blockIdx.x * n_eps + e) * T + t0 + r) * act_dim;
+                    float acc = 0.f;
+                    for (int j = 0; j < act_dim; ++j) acc = __fadd_rn(acc, __fmul_rn(__fadd_rn(a[j], __ldg(nz + j)), __ldg(c + j)));
+                    racc += (double)acc;
+                    if (e == n_eps - 1)
+                        for (int k = 0; k < 3; ++k) s_last[r][k] = __fadd_rn(a[k % act_dim], __ldg(nz + k % act_dim));
+                }
+                s_rew_e[r] = racc;
+            }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                double f = s_fit;
+                float p0 = s_pos[0], p1 = s_pos[1], p2 = s_pos[2];
+                for (int r = 0; r < rows; ++r) {
+                    f += s_rew_e[r];
+                    p0 = __fadd_rn(p0, __fmul_rn(pos_scale, s_last[r][0]));
+                    p1 = __fadd_rn(p1, __fmul_rn(pos_scale, s_last[r][1]));
+                    p2 = __fadd_rn(p2, __fmul_rn(pos_scale, s_last[r][2]));
+                }
+                s_fit = f; s_pos[0] = p0; s_pos[1] = p1; s_pos[2] = p2;
+            }
+            __syncthreads();
+            continue;
+        }
         if (act_noise) {
             // a += rs.randn(act) * ac_std (src/nn/nn.py:47-48): the scaled gaussians of this evaluation, drawn in stream order
             // by mt_gauss.cu; reward and position see the noisy action (the env receives it, gym_runner.py:53)
@@ -217,6 +254,7 @@ rollout_f32_kernel(const float* __restrict__ table, const int64_t* __restrict__ 
             }
         }
         if (writer) {
+            if (EPIS) f /= n_eps;                                        // obj.py: rews /= max(1, eps_per_policy)
             (neg ? fit_neg : fit_pos)[(size_t)pair * fit_stride] = f;
             float* b = neg ? behv_neg : behv_pos;
             if (b) { b[pair * 3 + 0] = p0; b[pair * 3 + 1] = p1; b[pair * 3 + 2] = p2; }
@@ -229,13 +267,13 @@ static int rf_round4(int x) { return (x + 3) & ~3; }
 int es_impl_rollout_f32(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
                         const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
                         const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
-                        float* behv_pos, float* behv_neg, const float* act_noise, cudaStream_t stream) {
+                        float* behv_pos, float* behv_neg, const float* act_noise, int n_eps, cudaStream_t stream) {
     // obs-64-64-act networks with enough pairs to fill the GPU: the packed-FMA kernel of rollout_f32x.cu (one CTA per pair);
     // fewer pairs than half the SMs (single evaluations, es.step's noiseless evaluation) stay here, where the episode's time
     // tiles are split over the idle SMs.  ES_F32_GENERAL=1 forces this kernel (tests compare the two).
     if (2 * n_pairs >= ctx->sm_count && !getenv("ES_F32_GENERAL")) {
         const int rc = es_impl_rollout_f32x(ctx, table, table_len, idx, n_pairs, theta, P, sigma, layer_sizes, n_layers, obsn, rew_vec,
-                                            T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg, act_noise, stream);
+                                            T, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos, behv_neg, act_noise, n_eps, stream);
         if (rc != ES_ERR_UNSUPPORTED) return rc;
     }
     RfDesc d;
@@ -307,18 +345,19 @@ int es_impl_rollout_f32(es_ctx* ctx, const float* table, int64_t table_len, cons
         double* fn = fit_neg + (size_t)p0 * fit_stride;
         float* bp = behv_pos ? behv_pos + (size_t)p0 * 3 : nullptr;
         float* bn = behv_neg ? behv_neg + (size_t)p0 * 3 : nullptr;
-        const float* an = act_noise ? act_noise + (size_t)p0 * 2 * T * layer_sizes[n_layers] : nullptr;
+        const float* an = act_noise ? act_noise + (size_t)p0 * 2 * n_eps * T * layer_sizes[n_layers] : nullptr;
         if (gw) {
             rollout_f32_stage_kernel<<<2 * np, RF_THREADS, 0, stream>>>(table, idx + p0, theta, sigma, d, wglobal);
             ES_LAUNCHED(ctx);
-            ES_CHECK_CUDA(cudaFuncSetAttribute(rollout_f32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)act_smem));
-            rollout_f32_kernel<true><<<dim3(2 * np, n_splits), RF_THREADS, act_smem, stream>>>(
-                table, idx + p0, theta, sigma, d, obsn, rew_vec, T, pos_scale, fp, fn, fit_stride, bp, bn, part, tickets, wglobal, an);
-        } else {
-            ES_CHECK_CUDA(cudaFuncSetAttribute(rollout_f32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));
-            rollout_f32_kernel<false><<<dim3(2 * np, n_splits), RF_THREADS, smem_w, stream>>>(
-                table, idx + p0, theta, sigma, d, obsn, rew_vec, T, pos_scale, fp, fn, fit_stride, bp, bn, part, tickets, nullptr, an);
         }
+        const dim3 grid(2 * np, n_splits);
+        const size_t smem = gw ? act_smem : smem_w;
+        const float* wg = gw ? wglobal : nullptr;
+        auto kernel = gw ? (n_eps > 1 ? rollout_f32_kernel<true, true> : rollout_f32_kernel<true, false>)
+                         : (n_eps > 1 ? rollout_f32_kernel<false, true> : rollout_f32_kernel<false, false>);
+        ES_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kernel<<<grid, RF_THREADS, smem, stream>>>(table, idx + p0, theta, sigma, d, obsn, rew_vec, T, pos_scale, fp, fn, fit_stride, bp,
+                                                   bn, part, tickets, wg, an, n_eps);
         ES_LAUNCHED(ctx);
     }
     return ES_OK;

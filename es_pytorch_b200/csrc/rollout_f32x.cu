@@ -67,6 +67,7 @@ struct FxParams {
     long long table_len;
     int P;
     int* err;
+    int n_eps;               // episodes per evaluation (act_noise [n_pairs][2][n_eps][T][act]); > 1 only in rollout_f32x_kernel<true>
 };
 
 struct FxSmem { uint32_t e1, xs, h, w2, w3, bias, posb, red, bars, total; int e1p, act4; };
@@ -169,6 +170,9 @@ __device__ __forceinline__ float fx_warp_sum8(const float (&v)[8], int lane) {
     return c;
 }
 
+// EPIS: p.n_eps > 1 episodes per evaluation sharing the forward pass; each adds its noise row to the layer-3 actions, its
+// float32 reward goes into the float64 sums, and the last one drives the position integrator
+template <bool EPIS>
 __global__ void __launch_bounds__(FX_THREADS, 1) rollout_f32x_kernel(const __grid_constant__ FxParams p) {
     extern __shared__ __align__(128) uint8_t fx_smem[];
     const FxSmem L = fx_layout(p.obs, p.act);
@@ -348,6 +352,31 @@ __global__ void __launch_bounds__(FX_THREADS, 1) rollout_f32x_kernel(const __gri
                     const bool unit = lane < p.act;
                     const float b3 = bias[sgn * (FX_H + 32) + FX_H + n3];
                     const int tb = m * FX_MT + r0;                                     // time step of row 0 of this warp
+                    if (EPIS) {
+                        float av[8], cw[8], v[8];
+#pragma unroll
+                        for (int a = 0; a < 8; ++a) {
+                            const bool live = unit && tb + a < p.T;
+                            av[a] = tanhf(fx_hsum(acc3[a]) + b3);
+                            cw[a] = live ? __ldg(p.rew + (size_t)(tb + a) * p.act + lane) : 0.f;
+                        }
+                        for (int e = 0; e < p.n_eps; ++e) {
+                            const float* __restrict__ nz = p.act_noise + ((((size_t)pair * 2 + sgn) * p.n_eps + e) * p.T + tb) * p.act + lane;
+#pragma unroll
+                            for (int a = 0; a < 8; ++a) {
+                                const bool live = unit && tb + a < p.T;
+                                const float ae = live ? __fadd_rn(av[a], __ldg(nz + a * p.act)) : 0.f;
+                                v[a] = ae * cw[a];
+                                if (want_pos && e == p.n_eps - 1) {
+#pragma unroll
+                                    for (int jj = 0; jj < 3; ++jj)
+                                        if (lane == jj % p.act) posb[(r0 + a) * 4 + jj] = ae;
+                                }
+                            }
+                            const float r = fx_warp_sum8(v, lane);         // lanes 4 q .. 4 q + 3: episode e's reward of row q
+                            if ((lane & 3) == 0) { if (sgn) fs1 += (double)r; else fs0 += (double)r; }
+                        }
+                    } else {
                     const float* __restrict__ nz = p.act_noise ? p.act_noise + (((size_t)pair * 2 + sgn) * p.T + tb) * p.act + lane : nullptr;
                     float v[8];
 #pragma unroll
@@ -364,6 +393,7 @@ __global__ void __launch_bounds__(FX_THREADS, 1) rollout_f32x_kernel(const __gri
                     }
                     const float r = fx_warp_sum8(v, lane);             // lanes 4 q .. 4 q + 3: the reward of row q
                     if ((lane & 3) == 0) { if (sgn) fs1 += (double)r; else fs0 += (double)r; }
+                    }
                 }
                 fx_bar();                                           // H is free again; the position columns are visible
                 if (want_pos && tid < 3) {
@@ -381,6 +411,7 @@ __global__ void __launch_bounds__(FX_THREADS, 1) rollout_f32x_kernel(const __gri
         if (tid == 0) {
             double fp = 0.0, fn = 0.0;
             for (int w = 0; w < FX_CWARPS; ++w) { fp += red[w * 2 + 0]; fn += red[w * 2 + 1]; }
+            if (EPIS) { fp /= p.n_eps; fn /= p.n_eps; }               // obj.py: rews /= max(1, eps_per_policy)
             p.fit_pos[(size_t)pair * p.fit_stride] = fp;
             p.fit_neg[(size_t)pair * p.fit_stride] = fn;
             if (want_pos) {
@@ -452,7 +483,7 @@ __global__ void __launch_bounds__(256) rollout_f32x_ubase_kernel(const float* __
 int es_impl_rollout_f32x(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
                          const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
                          const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
-                         float* behv_pos, float* behv_neg, const float* act_noise, cudaStream_t stream) {
+                         float* behv_pos, float* behv_neg, const float* act_noise, int n_eps, cudaStream_t stream) {
     if (n_layers != 3 || layer_sizes[1] != FX_H || layer_sizes[2] != FX_H || layer_sizes[3] > 32 || layer_sizes[0] < 1)
         return ES_ERR_UNSUPPORTED;
     const FxSmem L = fx_layout(layer_sizes[0], layer_sizes[3]);
@@ -466,7 +497,7 @@ int es_impl_rollout_f32x(es_ctx* ctx, const float* table, int64_t table_len, con
     p.n_tiles = es_div_up(T, FX_MT);
     p.sigma = sigma; p.pos_scale = pos_scale;
     p.w1 = 0; p.b1 = p.obs * FX_H; p.w2 = p.b1 + FX_H; p.b2 = p.w2 + FX_H * FX_H; p.w3 = p.b2 + FX_H; p.b3 = p.w3 + FX_H * p.act;
-    p.table_len = table_len; p.P = P; p.err = ctx->err_dev;
+    p.table_len = table_len; p.P = P; p.err = ctx->err_dev; p.n_eps = n_eps;
 
     const size_t xst_bytes = (size_t)p.n_tiles * p.nkc * FX_STAGE_FLOATS * sizeof(float);
     const size_t up_bytes = (size_t)p.n_tiles * 16 * FX_CT * sizeof(float);
@@ -486,8 +517,9 @@ int es_impl_rollout_f32x(es_ctx* ctx, const float* table, int64_t table_len, con
         ES_LAUNCHED(ctx);
     }
     const int grid = n_pairs < ctx->sm_count ? n_pairs : ctx->sm_count;
-    ES_CHECK_CUDA(cudaFuncSetAttribute(rollout_f32x_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));
-    rollout_f32x_kernel<<<grid, FX_THREADS, L.total, stream>>>(p);
+    auto kernel = n_eps > 1 ? rollout_f32x_kernel<true> : rollout_f32x_kernel<false>;
+    ES_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));
+    kernel<<<grid, FX_THREADS, L.total, stream>>>(p);
     ES_LAUNCHED(ctx);
     return ES_OK;
 }

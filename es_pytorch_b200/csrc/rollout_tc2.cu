@@ -140,9 +140,11 @@ static_assert(B2_COUNT * 8 + 16 <= 1024, "barrier block too small");
 
 // NOISE: the action-noise variant (loads of the noise array in the layer-3 epilogue); a separate instantiation so that the
 // registers it holds across the accumulator wait do not cost the noise-free kernel anything (measured: +6 % when shared)
-template <bool SPLIT, bool NOISE>
+// EPIS (with NOISE): n_eps > 1 episodes per evaluation, act_noise [n_pairs][2][n_eps][T][act]; the layer-3 epilogue keeps the
+// noise-free actions of its columns and adds every episode's noise row to them (the last episode drives the position)
+template <bool SPLIT, bool NOISE, bool EPIS>
 __global__ void __launch_bounds__(T2_THREADS, 1) rollout_tc2_kernel(const __grid_constant__ T2Params p,
-                                                                     const __grid_constant__ T2Maps maps) {
+                                                                     const __grid_constant__ T2Maps maps, int n_eps) {
     using C = T2Cfg<SPLIT>;
     constexpr int NP = C::NP, NST = C::NST;
     extern __shared__ uint8_t smem_raw[];
@@ -325,7 +327,18 @@ __global__ void __launch_bounds__(T2_THREADS, 1) rollout_tc2_kernel(const __grid
                 const int t = m * T2_MT + row;
                 const uint32_t tv_ = tmem + vbuf * C::V_STRIDE + lane_off + cq * CW;            // this warp's V columns
                 const float4* __restrict__ up = reinterpret_cast<const float4*>(p.ubase) + ((size_t)m * 16 + cq * (CW / 4)) * T2_MT + row;
-                if (NOISE && p.act_noise && cq == 0) {
+                if (EPIS && cq == 0) {
+                    // the noise rows of every episode of both signs ([sign][episode] blocks of T * act floats) towards L2
+                    const int t0 = m * T2_MT + q * 32;
+                    const int rows = min(32, p.T - t0);
+                    if (rows > 0) {
+                        const size_t blk = (size_t)p.T * p.act * 4;
+                        const char* nb = reinterpret_cast<const char*>(p.act_noise + (((size_t)(blockIdx.x + i * gridDim.x) * 2 * n_eps) * p.T + t0) * p.act);
+                        const int bytes = rows * p.act * 4;
+                        for (int k = 0; k < 2 * n_eps; ++k)
+                            for (int o = lane * 128; o < bytes + 128; o += 32 * 128) prefetch_l2(nb + k * blk + min(o, bytes - 4));
+                    }
+                } else if (NOISE && p.act_noise && cq == 0) {
                     // action noise of this tile's rows (both signs) towards L2 now; it is read after layer 3 (one warp per lane quarter asks)
                     const int t0 = m * T2_MT + q * 32;
                     const int rows = min(32, p.T - t0);
@@ -428,6 +441,61 @@ __global__ void __launch_bounds__(T2_THREADS, 1) rollout_tc2_kernel(const __grid
                 const float* nzrow = (NOISE && p.act_noise && t < p.T)
                     ? p.act_noise + (((size_t)(blockIdx.x + i * gridDim.x) * 2) * p.T + t) * p.act + a_lo : nullptr;
                 float tv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+                if (EPIS) {
+#pragma unroll
+                    for (int sgn = 0; sgn < 2; ++sgn) {
+                        mbar_wait(&bars[(sgn ? B2_D3N : B2_D3P) + eg], par);
+                        tc_fence_after();
+                        // a = tanh(D3 + b3) of this warp's columns, noise-free (padded columns: tanh(0), zero reward coefficient)
+                        float av[16];
+#pragma unroll
+                        for (int jj = 0; jj < 16; ++jj) av[jj] = 0.f;
+                        if (nj > 0) {
+                            const uint32_t b3 = sgn ? b3n : b3p;
+#pragma unroll
+                            for (int hf = 0; hf < 2; ++hf) {
+                                if (hf * 8 < nj) {
+                                    uint32_t d[8];
+                                    tmem_ld8(tb + (sgn ? C::C_D2N : C::C_D2P) + a_lo + hf * 8, d);      // D3 aliases D2
+                                    tmem_ld_wait();
+#pragma unroll
+                                    for (int g4 = 0; g4 < 2; ++g4) {
+                                        const int gq = hf * 2 + g4;
+                                        if (gq * 4 < nj) {
+                                            const float4 bb = lds128f(b3 + gq * 16);
+                                            const float z0 = __uint_as_float(d[g4 * 4 + 0]) + bb.x, z1 = __uint_as_float(d[g4 * 4 + 1]) + bb.y;
+                                            const float z2 = __uint_as_float(d[g4 * 4 + 2]) + bb.z, z3 = __uint_as_float(d[g4 * 4 + 3]) + bb.w;
+                                            float* a4 = av + gq * 4;
+                                            if (SPLIT) { tanh_acc2(z0, z1, a4[0], a4[1], (T2_NEWTON_MASK >> 0) & 1); tanh_acc2(z2, z3, a4[2], a4[3], (T2_NEWTON_MASK >> 1) & 1); }
+                                            else { a4[0] = tanh_fast(z0); a4[1] = tanh_fast(z1); a4[2] = tanh_fast(z2); a4[3] = tanh_fast(z3); }
+                                        }
+                                    }
+                                }
+                            }
+                        }
+                        tc_fence_before();
+                        if (t < p.T && nj > 0) {
+                            // episode e's noise row of this step and sign, columns a_lo..: obj.py's episode loop, one reward sum
+                            const float* __restrict__ ns =
+                                p.act_noise + ((((size_t)(blockIdx.x + i * gridDim.x) * 2 + sgn) * n_eps) * p.T + t) * p.act + a_lo;
+                            float r = 0.f, q0 = 0.f, q1 = 0.f, q2 = 0.f;
+                            for (int e = 0; e < n_eps; ++e) {
+                                const float* __restrict__ ne = ns + (size_t)e * p.T * p.act;
+                                float ae[16];
+#pragma unroll
+                                for (int jj = 0; jj < 16; ++jj) ae[jj] = av[jj] + ((jj < nj) ? ldg_pinned(ne + jj) : 0.f);
+#pragma unroll
+                                for (int jj = 0; jj < 16; ++jj) r = fmaf(ae[jj], cc[jj], r);
+                                q0 = ae[0]; q1 = (p.act > 1) ? ae[1] : ae[0]; q2 = (p.act > 2) ? ae[2] : ae[0];
+                            }
+                            // Kahan step: (s, c) += r
+                            if (sgn) { const float y = r - fnc, u = fns + y; fnc = (u - fns) - y; fns = u; tv[5] = q0; tv[6] = q1; tv[7] = q2; }
+                            else     { const float y = r - fpc, u = fps + y; fpc = (u - fps) - y; fps = u; tv[2] = q0; tv[3] = q1; tv[4] = q2; }
+                        }
+                    }
+                    if (want_pos && cq == 0) pacc += warp_sum8(tv, lane);
+                    continue;
+                }
                 // the noise values of a sign are in flight before that sign's accumulator is waited for (the - sign's under the
                 // + sign's arithmetic): read inside the tanh groups they cost several exposed memory latencies per tile
                 constexpr int NZ = NOISE ? (SPLIT ? 8 : 16) : 1;
@@ -517,6 +585,7 @@ __global__ void __launch_bounds__(T2_THREADS, 1) rollout_tc2_kernel(const __grid
                             for (int kk = 2; kk < 8; ++kk) tot[kk] += pf[kk];
                         }
                     }
+                    if (EPIS) { fp /= n_eps; fn /= n_eps; }                         // obj.py: rews /= max(1, eps_per_policy)
                     p.fit_pos[(size_t)pair * p.fit_stride] = fp;
                     p.fit_neg[(size_t)pair * p.fit_stride] = fn;
                     if (want_pos) {
@@ -777,7 +846,7 @@ int t2_encode_map(CUtensorMap* map, void* base, size_t stride, int obs) {
 
 template <bool SPLIT>
 int t2_launch(es_ctx* ctx, T2Params& p, const T2Maps& maps, const float* obsn, const float* rew_vec, const float* theta, int T,
-              int n_pairs, cudaStream_t stream) {
+              int n_pairs, int n_eps, cudaStream_t stream) {
     const T2Smem L = t2_layout<SPLIT>(p.nkc);
     const size_t smem = (size_t)L.total + 1024;       // + alignment slack
     if (smem > 227 * 1024) {
@@ -810,13 +879,10 @@ int t2_launch(es_ctx* ctx, T2Params& p, const T2Maps& maps, const float* obsn, c
         rollout_tc2_crt_kernel<<<es_div_up(p.n_mtiles * T2_ACT_PAD * T2_MT, 256), 256, 0, stream>>>(rew_vec, T, p.act, p.n_mtiles, crt);
         ES_LAUNCHED(ctx);
     }
-    if (p.act_noise) {
-        ES_CHECK_CUDA(cudaFuncSetAttribute(rollout_tc2_kernel<SPLIT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        rollout_tc2_kernel<SPLIT, true><<<grid, T2_THREADS, smem, stream>>>(p, maps);
-    } else {
-        ES_CHECK_CUDA(cudaFuncSetAttribute(rollout_tc2_kernel<SPLIT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        rollout_tc2_kernel<SPLIT, false><<<grid, T2_THREADS, smem, stream>>>(p, maps);
-    }
+    auto kernel = !p.act_noise ? rollout_tc2_kernel<SPLIT, false, false>
+                               : (n_eps > 1 ? rollout_tc2_kernel<SPLIT, true, true> : rollout_tc2_kernel<SPLIT, true, false>);
+    ES_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, T2_THREADS, smem, stream>>>(p, maps, n_eps);
     ES_LAUNCHED(ctx);
     return ES_OK;
 }
@@ -835,7 +901,7 @@ void es_tc2_free_shadows(es_ctx* ctx) {
 int es_impl_rollout_tc2(es_ctx* ctx, int split, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
                         const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
                         const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
-                        float* behv_pos, float* behv_neg, const float* act_noise, cudaStream_t stream) {
+                        float* behv_pos, float* behv_neg, const float* act_noise, int n_eps, cudaStream_t stream) {
     if (n_layers != 3 || layer_sizes[1] != T2_H || layer_sizes[2] != T2_H || layer_sizes[3] > T2_ACT_PAD || layer_sizes[0] > 1023) {
         es_set_error("es_rollout_openloop(TC): the tensor-core path covers obs(<=1023)-64-64-act(<=32) tanh MLPs; "
                      "use ES_ROLLOUT_F32 for other shapes");
@@ -901,6 +967,6 @@ int es_impl_rollout_tc2(es_ctx* ctx, int split, const float* table, int64_t tabl
             p.shadow_stride = stride;
         }
     }
-    return split ? t2_launch<true>(ctx, p, maps, obsn, rew_vec, theta, T, n_pairs, stream)
-                 : t2_launch<false>(ctx, p, maps, obsn, rew_vec, theta, T, n_pairs, stream);
+    return split ? t2_launch<true>(ctx, p, maps, obsn, rew_vec, theta, T, n_pairs, n_eps, stream)
+                 : t2_launch<false>(ctx, p, maps, obsn, rew_vec, theta, T, n_pairs, n_eps, stream);
 }

@@ -60,9 +60,12 @@ struct TwParams {
     long long table_len;
     int P;
     int* err;
+    int n_eps;                    // episodes per evaluation (act_noise [n_pairs][2][n_eps][T][act]); > 1 only with EPIS
 };
 
-template <bool SPLIT>
+// EPIS: p.n_eps > 1 episodes per evaluation sharing the forward pass; the output epilogue adds every episode's noise row to the
+// noise-free actions, sums each episode's float32 reward into the float64 fitness, and integrates the last episode's position
+template <bool SPLIT, bool EPIS>
 __global__ void __launch_bounds__(TW_THREADS, 1) rollout_tcw_kernel(const __grid_constant__ TwParams p) {
     constexpr int NP = SPLIT ? 2 : 1;
     extern __shared__ uint8_t smem_raw[];
@@ -256,7 +259,32 @@ __global__ void __launch_bounds__(TW_THREADS, 1) rollout_tcw_kernel(const __grid
                                 if (SPLIT) tanh_acc2(z0, z1, a[2 * e], a[2 * e + 1], false);
                                 else { a[2 * e] = tanh_fast(z0); a[2 * e + 1] = tanh_fast(z1); }
                             }
-                            if (t < p.T) {
+                            if (EPIS && t < p.T) {
+                                const float* __restrict__ c = p.rew_vec + (size_t)t * act;
+                                const float* __restrict__ ns = p.act_noise + ((((size_t)pair * 2 + s) * p.n_eps) * p.T + t) * act;
+                                float cw[8], ae[8];
+#pragma unroll
+                                for (int e = 0; e < 8; ++e) cw[e] = (cq * 8 + e < act) ? __ldg(c + cq * 8 + e) : 0.f;
+                                for (int ep = 0; ep < p.n_eps; ++ep) {
+                                    const float* __restrict__ nz = ns + (size_t)ep * p.T * act;
+                                    float r = 0.f;
+#pragma unroll
+                                    for (int e = 0; e < 8; ++e) {
+                                        const int j = cq * 8 + e;
+                                        ae[e] = a[e];
+                                        if (j < act) {
+                                            ae[e] = __fadd_rn(a[e], __ldg(nz + j));
+                                            r = __fadd_rn(r, __fmul_rn(ae[e], cw[e]));
+                                        }
+                                    }
+                                    fit[s] += (double)r;
+                                }
+                                if (cq == 0) {                                  // the last episode's position
+                                    pos[3 * s + 0] += (double)ae[0];
+                                    pos[3 * s + 1] += (double)(act > 1 ? ae[1] : ae[0]);
+                                    pos[3 * s + 2] += (double)(act > 2 ? ae[2] : ae[0]);
+                                }
+                            } else if (!EPIS && t < p.T) {
                                 const float* __restrict__ c = p.rew_vec + (size_t)t * act;
                                 const float* __restrict__ nz =
                                     p.act_noise ? p.act_noise + (((size_t)pair * 2 + s) * p.T + t) * act : nullptr;
@@ -283,6 +311,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) rollout_tcw_kernel(const __grid
                     }
             }
             // this warp's sums of the pair -> shared memory (butterfly: the same order on every run)
+            if (EPIS) { fit[0] /= p.n_eps; fit[1] /= p.n_eps; }       // obj.py: rews /= max(1, eps_per_policy)
             double w8[8] = {fit[0], fit[1], pos[0], pos[1], pos[2], pos[3], pos[4], pos[5]};
 #pragma unroll
             for (int k = 0; k < 8; ++k) w8[k] = warp_sum_d(w8[k]);
@@ -315,6 +344,7 @@ __global__ void __launch_bounds__(TW_THREADS, 1) rollout_tcw_kernel(const __grid
 
 template <bool SPLIT>
 int tw_launch(es_ctx* ctx, TwParams& p, const float* obsn, int T, int n_pairs, cudaStream_t stream) {
+    auto kernel = p.n_eps > 1 ? rollout_tcw_kernel<SPLIT, true> : rollout_tcw_kernel<SPLIT, false>;
     constexpr int NP = SPLIT ? 2 : 1;
     int nmax = 0, bias_floats = 0;
     uint32_t img = 0;
@@ -357,8 +387,8 @@ int tw_launch(es_ctx* ctx, TwParams& p, const float* obsn, int T, int n_pairs, c
         rollout_tc2_prep_kernel<SPLIT><<<blocks, 256, 0, stream>>>(obsn, T, p.in[0], p.nkc[0], p.n_mtiles, xnt);
         ES_LAUNCHED(ctx);
     }
-    ES_CHECK_CUDA(cudaFuncSetAttribute(rollout_tcw_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    rollout_tcw_kernel<SPLIT><<<grid, TW_THREADS, smem, stream>>>(p);
+    ES_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, TW_THREADS, smem, stream>>>(p);
     ES_LAUNCHED(ctx);
     return ES_OK;
 }
@@ -376,7 +406,7 @@ int es_tcw_covers(const int* layer_sizes, int n_layers) {
 int es_impl_rollout_tcw(es_ctx* ctx, int split, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
                         const float* theta, int P, float sigma, const int* layer_sizes, int n_layers, const float* obsn,
                         const float* rew_vec, int T, float pos_scale, double* fit_pos, double* fit_neg, int fit_stride,
-                        float* behv_pos, float* behv_neg, const float* act_noise, cudaStream_t stream) {
+                        float* behv_pos, float* behv_neg, const float* act_noise, int n_eps, cudaStream_t stream) {
     if (!es_tcw_covers(layer_sizes, n_layers)) {
         es_set_error("es_rollout_openloop(TC): the wide tensor-core path covers obs(<=1023) -> 2..4 hidden layers (multiples of "
                      "64 in [64, 256]) -> act(<=32) tanh MLPs");
@@ -398,6 +428,6 @@ int es_impl_rollout_tcw(es_ctx* ctx, int split, const float* table, int64_t tabl
         p.b_off[l] = off; off += p.out[l];
     }
     p.sigma = sigma; p.pos_scale = pos_scale;
-    p.table_len = table_len; p.P = P; p.err = ctx->err_dev;
+    p.table_len = table_len; p.P = P; p.err = ctx->err_dev; p.n_eps = n_eps;
     return split ? tw_launch<true>(ctx, p, obsn, T, n_pairs, stream) : tw_launch<false>(ctx, p, obsn, T, n_pairs, stream);
 }

@@ -247,8 +247,23 @@ class Engine:
     # ------------------------------------------------------------------ a3+a4+a5
     def rollout(self, table, idx, theta, sigma: float, layer_sizes: Sequence[int], obsn, rew_vec, pos_scale: float,
                 fit_pos, fit_neg, fit_stride: int = 1, behv_pos=None, behv_neg=None, mode: int = ES_ROLLOUT_F32,
-                act_noise=None):
-        """``act_noise``: float32 [n_pairs, 2, T, act] scaled action noise (``draw_noisy``), added to every action."""
+                act_noise=None, n_episodes: int = 1):
+        """``act_noise``: float32 [n_pairs, 2, n_episodes, T, act] scaled action noise (``draw_noisy``), added to every
+        action.  ``n_episodes`` > 1: every evaluation is that many episodes (obj.py's eps_per_policy), each with its own
+        noise; fitness = their per-step average summed, behaviour = the last episode's (``rollout_episodes``)."""
+        self._rollout(table, idx, theta, sigma, layer_sizes, obsn, rew_vec, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos,
+                      behv_neg, mode, act_noise, n_episodes, n_episodes != 1)
+
+    def rollout_episodes(self, table, idx, theta, sigma: float, layer_sizes: Sequence[int], obsn, rew_vec, pos_scale: float,
+                         fit_pos, fit_neg, fit_stride: int = 1, behv_pos=None, behv_neg=None, mode: int = ES_ROLLOUT_F32,
+                         act_noise=None, n_episodes: int = 1):
+        """es_rollout_openloop_episodes for any ``n_episodes`` (``rollout`` takes es_rollout_openloop_noisy for one episode;
+        both give the same results then).  The library rejects n_episodes < 1 and n_episodes * T * act > INT_MAX."""
+        self._rollout(table, idx, theta, sigma, layer_sizes, obsn, rew_vec, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos,
+                      behv_neg, mode, act_noise, n_episodes, True)
+
+    def _rollout(self, table, idx, theta, sigma, layer_sizes, obsn, rew_vec, pos_scale, fit_pos, fit_neg, fit_stride, behv_pos,
+                 behv_neg, mode, act_noise, n_episodes, episodes_entry):
         d = self.device
         _req(table, torch.float32, 'table', d); _req(idx, torch.int64, 'idx', d); _req(theta, torch.float32, 'theta', d)
         _req(obsn, torch.float32, 'obsn', d); _req(rew_vec, torch.float32, 'rew_vec', d)
@@ -262,7 +277,7 @@ class Engine:
             assert behv_pos.numel() == 3 * n and behv_neg.numel() == 3 * n
         if act_noise is not None:
             _req(act_noise, torch.float32, 'act_noise', d)
-            assert act_noise.numel() == n * 2 * T * layer_sizes[-1]
+            assert n_episodes < 1 or act_noise.numel() == n * 2 * int(n_episodes) * T * layer_sizes[-1]
         ls = (C.c_int * len(layer_sizes))(*[int(x) for x in layer_sizes])
         if mode in (ES_ROLLOUT_TC, ES_ROLLOUT_TC3):
             # the library keeps a bf16 shadow of the table keyed by (pointer, length); a different tensor object (the
@@ -271,6 +286,13 @@ class Engine:
             if ref is None or ref() is not table or ver != table._version:
                 check(self.lib.es_noise_table_changed(self._ctx), 'es_noise_table_changed')
                 self._tc_table = (weakref.ref(table), table._version)
+        if episodes_entry:
+            check(self.lib.es_rollout_openloop_episodes(self._ctx, _ptr(table), table.numel(), _ptr(idx), n, _ptr(theta),
+                                                        theta.numel(), float(sigma), ls, len(layer_sizes) - 1, _ptr(obsn),
+                                                        _ptr(rew_vec), T, float(pos_scale), _ptr(fit_pos), _ptr(fit_neg),
+                                                        int(fit_stride), _ptr(behv_pos), _ptr(behv_neg), _ptr(act_noise),
+                                                        int(n_episodes), int(mode), self.stream), 'es_rollout_openloop_episodes')
+            return
         check(self.lib.es_rollout_openloop_noisy(self._ctx, _ptr(table), table.numel(), _ptr(idx), n, _ptr(theta),
                                                  theta.numel(), float(sigma), ls, len(layer_sizes) - 1, _ptr(obsn),
                                                  _ptr(rew_vec), T, float(pos_scale), _ptr(fit_pos), _ptr(fit_neg),

@@ -71,7 +71,7 @@ class DeviceGeneration:
                  optim: Optimizer, ob_clip: float = 5.0, pos_scale: float = 0.05, coins_per_eval: int = 0,
                  save_obs_chance: float = 0.0, archive: Optional[torch.Tensor] = None, nov_k: int = 10,
                  moo_w: float = 1.0, rollout_mode: int = ES_ROLLOUT_F32, comm: Optional[dist.Comm] = None,
-                 engine: Optional[Engine] = None, ranker=None, ac_std: float = 0.0, closed=None):
+                 engine: Optional[Engine] = None, ranker=None, ac_std: float = 0.0, closed=None, eps_per_policy: int = 1):
         self.eng = engine or get_engine()
         # closed-loop variant of the synthetic env (gym.synthetic_env.ClosedLoopEnv): (obs_0 [obs], A^T [band, obs], B^T [act, obs]);
         # row 0 of obs_stream is then the only one read and the rollout is es_rollout_closedloop
@@ -97,6 +97,9 @@ class DeviceGeneration:
         # FeedForward._action_std (nn.py:47-48): != 0 -> every step adds rs.randn(act) * ac_std, drawn from the rank streams
         self.ac_std = float(ac_std or 0.0)
         self.act_noise = None
+        # episodes per evaluation (obj.py's eps_per_policy): each draws its own T * act gaussians after the coin; on the open-loop
+        # env they share the forward pass (es_rollout_openloop_episodes).  Without action noise they are all the same episode.
+        self.eps_per_policy = max(1, int(eps_per_policy))
         assert self.coins_per_eval in (0, 1), 'fit_fns draw at most one save_obs coin per evaluation'
 
         # per-rank MT19937 streams, resident on the device between generations
@@ -188,8 +191,9 @@ class DeviceGeneration:
         self.version += 1
         with self._timed('draw_indices'):
             if self.ac_std != 0.0:
-                # indices, coins and the action noise of every rollout, in the reference's stream order (mt_gauss.cu)
-                nrm = self.T * self.act_dim
+                # indices, coins and the action noise of every rollout, in the reference's stream order (mt_gauss.cu); the
+                # E episodes of an evaluation are E * T * act consecutive gaussians after its coin
+                nrm = self.eps_per_policy * self.T * self.act_dim
                 if self.act_noise is None or self.act_noise.shape != (self.k_local, 2, nrm):
                     self.act_noise = e.empty((self.k_local, 2, nrm), torch.float32)
                 e.draw_noisy(self.mt_key, self.mt_pos, self.mt_has, self.mt_gauss, n_per_stream, self.table.numel() - self.P,
@@ -237,7 +241,8 @@ class DeviceGeneration:
             e.rollout(self.table, self.idx, self.theta, self.sigma, self.layer_sizes, self.obsn, self.rew_vec,
                       self.pos_scale, fp, fn, self.n_obj, None if self.behv is None else self.behv[0],
                       None if self.behv is None else self.behv[1], self.rollout_mode,
-                      act_noise=self.act_noise if self.ac_std != 0.0 else None)
+                      act_noise=self.act_noise if self.ac_std != 0.0 else None,
+                      n_episodes=self.eps_per_policy if self.ac_std != 0.0 else 1)
         if self.n_obj == 2:
             # second objective column = novelty of the final (x, y) (training_result.py:95-97)
             e.novelty(self.behv.view(-1, 3), self.archive, self.nov_k, self.fit_local.view(-1)[1:], 2)

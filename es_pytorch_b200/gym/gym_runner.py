@@ -35,7 +35,9 @@ def hbaselines_pos(env):
     return tuple(env.wrapped_env.get_body_com('torso')[:3])
 
 
-def _device_episode(model, env, max_steps: int, rs=None):
+def _device_episode(model, env, max_steps: int, rs=None, n_episodes: int = 1):
+    """``n_episodes`` > 1 (obj.py's eps_per_policy): that many episodes with their own action noise, one launch of
+    es_rollout_openloop_episodes; the total is their per-step average summed, the position the last episode's."""
     from ..engine import get_engine
     from ..core.policy import Policy
     eng = get_engine()
@@ -53,14 +55,16 @@ def _device_episode(model, env, max_steps: int, rs=None):
     behv = torch.zeros(2, 3, dtype=torch.float32, device=eng.device)
     noise = None
     ac_std = float(getattr(model, '_action_std', 0) or 0)
+    E = 1
     if rs is not None and ac_std != 0:
         # nn.py:47-48: T calls of rs.randn(act) * ac_std; one call of rs.randn(T * act) consumes the stream identically
-        # (legacy gaussians are produced one by one, cached second value included).  [pair 0][+ | -][T][act]: both
-        # evaluations of the sigma = 0 "pair" see the same noise, only the first is used.
-        nz = (rs.randn(T * sizes[-1]) * ac_std).astype(np.float32)
+        # (legacy gaussians are produced one by one, cached second value included); E episodes in a row: rs.randn(E * T * act).
+        # [pair 0][+ | -][E][T][act]: both evaluations of the sigma = 0 "pair" see the same noise, only the first is used.
+        E = max(1, int(n_episodes))
+        nz = (rs.randn(E * T * sizes[-1]) * ac_std).astype(np.float32)
         noise = eng.to_device(np.stack([nz, nz]).reshape(1, 2, -1))
     eng.rollout(table, idx, theta, 0.0, sizes, obsn, rew_dev[:T].contiguous(), env.pos_scale, fit[0:1], fit[1:2], 1,
-                behv[0:1].view(-1), behv[1:2].view(-1), act_noise=noise)
+                behv[0:1].view(-1), behv[1:2].view(-1), act_noise=noise, n_episodes=E)
     return float(fit[0].item()), behv[0].cpu().numpy().astype(np.float64), T
 
 

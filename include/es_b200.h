@@ -123,6 +123,21 @@ int es_rollout_openloop_noisy(es_ctx* ctx, const float* table, int64_t table_len
                               double* fit_pos, double* fit_neg, int fit_stride, float* behv_pos, float* behv_neg,
                               const float* act_noise, int mode, void* stream);
 
+/* The same with n_episodes >= 1 episodes per evaluation (obj.py's r_fn: `for _ in range(max(1, eps_per_policy))` runs the
+ * policy E times, adds the per-step rewards in a float64 array and divides it by E; behaviour = the last episode's).  On the
+ * open-loop env the E episodes share their forward pass and differ only in the action noise:
+ *   act_noise dev float [n_pairs][2 (+,-)][n_episodes][T][act_dim] (es_draw_noisy with normals_per_eval = n_episodes*T*act_dim)
+ *   fitness   = (sum over steps and episodes of the float32 reward of episode e's noisy action, in float64) / n_episodes
+ *   behv      = the final position of episode n_episodes - 1
+ * With act_noise == NULL every episode is the noise-free one and the call is es_rollout_openloop (exact: the reference's
+ * per-step average of E equal float32 rewards is that reward).  n_episodes * T * act_dim must not exceed INT_MAX
+ * (ES_ERR_INVALID), the noise offsets are 64-bit.  n_episodes == 1 is es_rollout_openloop_noisy.                       */
+int es_rollout_openloop_episodes(es_ctx* ctx, const float* table, int64_t table_len, const int64_t* idx, int n_pairs,
+                                 const float* theta, int P, float sigma, const int* layer_sizes, int n_layers,
+                                 const float* obsn, const float* rew_vec, int T, float pos_scale,
+                                 double* fit_pos, double* fit_neg, int fit_stride, float* behv_pos, float* behv_neg,
+                                 const float* act_noise, int n_episodes, int mode, void* stream);
+
 /* ---- a3 + a4 + a5 on the CLOSED-LOOP synthetic env (SURVEY.md section 8d's optional variant; never part of the headline) --
  * obs_{t+1} = tanh(A obs_t + B a_t): the observation depends on the policy's own actions, so the episode runs step by step
  * with one pair's perturbed weights resident on chip (rollout_closed.cu).  Replaces the same reference loop as
